@@ -18,6 +18,11 @@ default `--modes auto`, a `modes` block with the other BASELINE.json configs mea
 so every reference-vs-ours row comes from the same box and the same launch.  At N > 1 our arm also emits `comm_check`:
 our NVLS all-reduce / reduce-to-owner / broadcast kernels against NCCL on 3 KB / 2.4 MB / 77 MB buffers, and a bitwise
 comparison of the replicas' parameters after the timed steps.
+
+`--dump-outputs DIR` (our arm) writes what the headline config's last timed step produced, as float32 `.npy` files: `loss`,
+and for every parameter `param.<name>` (the model's weights) and `master.<name>` (the fp32 master copy, bf16 runs).
+Tensors above DUMP_SAMPLE elements are reduced to a fixed sample of positions seeded by the array's name, so two builds run
+with the same arguments can be compared file by file; rank 0 writes.
 """
 from __future__ import annotations
 
@@ -40,6 +45,8 @@ MODEL_DIMS = {"tiny": (2, 2, 128), "small": (12, 12, 768), "medium": (24, 16, 10
 EXTRA_MODES = [("zero1", "medium"), ("zero2", "large"), ("zero3", "xl")]
 OPTIMIZER_DESC = "AdamW lr1e-5 wd0.1 (coupled L2)"
 L2_DESC = "working set (params+grads+optimizer state, GBs) >> 126 MB L2; no explicit flush"
+DUMP_SAMPLE = 65536            # elements kept per dumped array
+DUMP_BUDGET = 12 << 20         # elements over all dumped arrays (48 MB of float32)
 
 
 def parse():
@@ -61,6 +68,8 @@ def parse():
     ap.add_argument("--modes", default="auto", choices=["auto", "none", "all"],
                     help="auto: add the zero1-medium / zero2-large / zero3-xl block when the headline is the default ddp-small")
     ap.add_argument("--mode-steps", type=int, default=10, help="timed steps of each extra config in the `modes` block")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="our arm: write the loss and (sampled) parameters of the last timed step as DIR/<name>.npy (float32)")
     return ap.parse_args()
 
 
@@ -211,6 +220,31 @@ def free_cuda():
     torch.cuda.reset_peak_memory_stats()
 
 
+def dump_outputs(out_dir, loss, opt):
+    """Write the step's loss, every non-empty parameter and its fp32 master copy (where the optimizer keeps one) as float32
+    ``out_dir/<name>.npy``.  Arrays longer than the per-array share of DUMP_BUDGET (at most DUMP_SAMPLE) keep the same
+    sorted sample of flat positions on every run: the sampler is seeded by the array's name.  Returns the names written."""
+    import zlib
+    import numpy as np
+    import torch
+    arrays = {"loss": loss.detach().reshape(1)}
+    for name, p in opt.parameters.items():
+        if p.numel():
+            arrays[f"param.{name}"] = p.detach()
+        master = opt.state.get(name, {}).get("master")
+        if master is not None and master.numel():
+            arrays[f"master.{name}"] = master
+    keep = min(DUMP_SAMPLE, DUMP_BUDGET // len(arrays))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        flat = t.reshape(-1)
+        if flat.numel() > keep:
+            pos = np.random.default_rng(zlib.crc32(name.encode())).choice(flat.numel(), size=keep, replace=False)
+            flat = flat[torch.from_numpy(np.sort(pos)).to(flat.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), flat.float().cpu().numpy())
+    return list(arrays)
+
+
 # ------------------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------------------
@@ -251,8 +285,9 @@ def build_ours(args, mode, model_name, rank, world, device):
 
 
 def measure_ours(args, mode, model_name, steps, warmup, rank, local, world, device, *, with_e2e=True, with_exposed=True,
-                 keep=None, check_replicas=False):
-    """One config through the public API (TrainStep).  Returns the result dict (same on every rank)."""
+                 keep=None, check_replicas=False, dump_dir=None):
+    """One config through the public API (TrainStep).  Returns the result dict (same on every rank).  With ``dump_dir``,
+    rank 0 writes the outputs of the last device-timed step there (dump_outputs)."""
     import torch
     import tiny_deepspeed_b200 as tds
     from tiny_deepspeed_b200 import ops
@@ -290,6 +325,8 @@ def measure_ours(args, mode, model_name, steps, warmup, rank, local, world, devi
     barrier_sync(device)
     ms_step = max_over_ranks(e0.elapsed_time(e1), device) / steps
     final_loss = float(loss.item())
+    if dump_dir is not None and rank == 0:
+        dump_outputs(dump_dir, loss, opt)
 
     # ---- end-to-end arm: public API call per step, pinned-host inputs in, loss out ----------------------
     e2e_ms = None
@@ -424,7 +461,7 @@ def run_ours(args):
     rank, local, world, device = setup_dist(args)
     keep = {}
     head = measure_ours(args, args.mode, args.model, args.steps, args.warmup, rank, local, world, device, keep=keep,
-                        check_replicas=True)
+                        check_replicas=True, dump_dir=args.dump_outputs)
     check = None
     if world > 1:
         try:
@@ -445,7 +482,7 @@ def run_ours(args):
         for mode, model_name in EXTRA_MODES:
             key = f"{mode}-{model_name}"
             try:
-                r = measure_ours(args, mode, model_name, max(3, min(args.steps, args.mode_steps)), min(max(args.warmup, 3), 4),
+                r = measure_ours(args, mode, model_name, min(args.steps, args.mode_steps), min(max(args.warmup, 3), 4),
                                  rank, local, world, device, with_e2e=False)
                 modes[key] = {k: r[k] for k in ("config", "value", "ms_per_step", "final_loss", "peak_hbm_bytes",
                                                "exposed_comm_ms_per_step", "launches_per_step", "backend", "steps", "warmup")}
@@ -579,7 +616,7 @@ def run_reference(args):
             for mode, model_name in EXTRA_MODES:
                 key = f"{mode}-{model_name}"
                 try:
-                    r = measure_reference(args, mode, model_name, max(3, min(args.steps, args.mode_steps)),
+                    r = measure_reference(args, mode, model_name, min(args.steps, args.mode_steps),
                                           min(max(args.warmup, 3), 4), rank, local, world, device, with_e2e=False)
                     modes[key] = {k: r[k] for k in ("config", "value", "ms_per_step", "final_loss", "peak_hbm_bytes",
                                                    "steps", "warmup")}

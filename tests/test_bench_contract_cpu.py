@@ -62,5 +62,45 @@ def test_round2_lines_carry_modes_and_comm_check():
 def test_bench_cli_parses_on_cpu():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--help"], capture_output=True, text=True, timeout=120)
     assert r.returncode == 0
-    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--dtype", "--mode"):
+    for flag in ("--gpus", "--steps", "--warmup", "--impl", "--dtype", "--mode", "--dump-outputs"):
         assert flag in r.stdout
+
+
+def test_dump_outputs_writes_float32_sampled_reproducible_arrays(tmp_path, monkeypatch):
+    """bench.dump_outputs: loss + every parameter + its fp32 master as float32 .npy, long arrays cut to the per-array share
+    of the budget at name-seeded positions, so two dumps of the same state are identical."""
+    import importlib.util
+    import numpy as np
+    import torch
+    import tiny_deepspeed_b200 as tds
+    from tiny_deepspeed_b200.models.gpt2 import GPT2Model, gpt2_config
+
+    spec = importlib.util.spec_from_file_location("bench_under_test", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    monkeypatch.setattr(bench, "DUMP_SAMPLE", 1000)
+    monkeypatch.setattr(bench, "DUMP_BUDGET", 20000)
+    torch.manual_seed(0)
+    model = GPT2Model(gpt2_config("tiny")).to(torch.bfloat16)
+    opt = tds.AdamW(model.named_parameters(), lr=1e-3)
+    names = bench.dump_outputs(str(tmp_path / "a"), torch.tensor(2.5), opt)
+    assert bench.dump_outputs(str(tmp_path / "b"), torch.tensor(2.5), opt) == names
+    params = dict(model.named_parameters())
+    assert names[0] == "loss"
+    assert sorted(names[1:]) == sorted([f"param.{n}" for n in params] + [f"master.{n}" for n in params])
+    keep = min(1000, 20000 // len(names))
+    total = 0
+    for n in names:
+        a, b = np.load(tmp_path / "a" / f"{n}.npy"), np.load(tmp_path / "b" / f"{n}.npy")
+        assert a.dtype == np.float32 and a.ndim == 1 and np.array_equal(a, b), n
+        total += a.size
+        if n == "loss":
+            assert a.tolist() == [2.5]
+            continue
+        src = params[n.split(".", 1)[1]].detach().float().reshape(-1).numpy()
+        assert a.size == min(src.size, keep), n
+        if src.size <= keep:
+            assert np.array_equal(a, src), n
+        else:
+            assert np.isin(a, src).all(), n
+    assert total <= 20000

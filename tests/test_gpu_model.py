@@ -62,6 +62,36 @@ def test_smoke_entry():
     g.smoke()
 
 
+def test_bench_dump_outputs_reproducible(tmp_path):
+    """bench.py --dump-outputs end to end (tiny model): the JSON line reports the requested steps, loss.npy is the reported
+    final loss, and a second run with the same arguments dumps the same arrays (up to atomics-order rounding)."""
+    import json
+    import os
+    import subprocess
+    import sys
+    import numpy as np
+    from dist_utils import free_port
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    runs = []
+    for tag in ("a", "b"):
+        out = tmp_path / tag
+        r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--model", "tiny", "--modes", "none", "--steps", "3",
+                            "--warmup", "2", "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600,
+                           env={**os.environ, "MASTER_PORT": str(free_port())})
+        assert r.returncode == 0, r.stderr[-2000:]
+        line = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][-1])
+        assert line["steps"] == 3
+        loss = np.load(out / "loss.npy")
+        assert loss.dtype == np.float32 and loss.tolist() == [pytest.approx(line["final_loss"], rel=1e-6)]
+        runs.append({p.stem: np.load(p) for p in out.glob("*.npy")})
+    a, b = runs
+    assert set(a) == set(b) and any(k.startswith("master.") for k in a) and sum(v.nbytes for v in a.values()) <= 64 << 20
+    for k in a:
+        assert a[k].dtype == np.float32 and np.isfinite(a[k]).all(), k
+        np.testing.assert_allclose(a[k], b[k], rtol=1e-3, atol=1e-3, err_msg=k)
+
+
 def test_optimizer_in_backward_overlap_matches_plain_step():
     cfg, m1 = _mk(2)
     m2 = copy.deepcopy(m1)
