@@ -133,7 +133,8 @@ std::vector<Tensor> layernorm_fwd_(const Tensor& x, const Tensor& w, const Tenso
   c10::cuda::CUDAGuard guard(x.device());
   TORCH_CHECK(x.dim() == 2 && x.is_contiguous() && w.is_contiguous() && b.is_contiguous());
   const int M = x.size(0), N = x.size(1);
-  TORCH_CHECK(N % 8 == 0 || true);
+  TORCH_CHECK(w.numel() == N && b.numel() == N && w.scalar_type() == x.scalar_type() && b.scalar_type() == x.scalar_type(),
+              "layernorm_fwd: weight and bias must be [N] of the input's dtype");
   Tensor y = torch::empty_like(x);
   auto fopt = x.options().dtype(at::kFloat);
   Tensor mean = torch::empty({M}, fopt), rstd = torch::empty({M}, fopt);
@@ -160,7 +161,8 @@ Tensor layernorm_bwd_(const Tensor& dy, const Tensor& x, const Tensor& w, const 
   // ln_fold_kernel, deterministic summation order) — 128 CTAs finishing together serialise in the L2 atomic units.
   static const bool deterministic = !(getenv("TDS_LN_SINGLE") && atoi(getenv("TDS_LN_SINGLE")) != 0);
   const bool want_single = variant < 0 ? !deterministic : variant == 1;
-  const bool single = want_single && x.scalar_type() == at::kBFloat16 && N % 8 == 0 && N <= 2048;
+  const bool single = want_single && layernorm_bwd_fast_ok(dy.data_ptr(), x.data_ptr(), w.data_ptr(), addp, dx.data_ptr(), N,
+                                                           dtype_of(x));
   static std::vector<Tensor> counters(64), accs(64);
   const int dev = x.get_device();
   Tensor scratch;

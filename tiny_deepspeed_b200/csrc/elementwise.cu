@@ -36,7 +36,8 @@ template <> struct V8<float> {
 // =====================================================================================================
 constexpr int kLnWarps = 4;
 
-template <typename T>
+// VEC: the 16-byte path is legal for this launch (rows_vec16); otherwise the scalar tail loops cover the whole row.
+template <typename T, bool VEC>
 __global__ void __launch_bounds__(kLnWarps * 32) ln_fwd_kernel(const T* __restrict__ x, const T* __restrict__ w,
                                                               const T* __restrict__ b, T* __restrict__ y,
                                                               float* __restrict__ mean, float* __restrict__ rstd,
@@ -47,7 +48,7 @@ __global__ void __launch_bounds__(kLnWarps * 32) ln_fwd_kernel(const T* __restri
   if (row >= M) return;
   const T* xr = x + (size_t)row * N;
   T* yr = y + (size_t)row * N;
-  const int nvec = N >> 3;
+  const int nvec = VEC ? N >> 3 : 0;
   float s = 0.f;
   for (int i = lane; i < nvec; i += 32) {
     float f[8];
@@ -82,8 +83,9 @@ __global__ void __launch_bounds__(kLnWarps * 32) ln_fwd_kernel(const T* __restri
 void layernorm_fwd(const void* x, const void* w, const void* b, void* y, float* mean, float* rstd, int M, int N,
                    float eps, int dtype, cudaStream_t s) {
   dim3 grid((M + kLnWarps - 1) / kLnWarps), block(kLnWarps * 32);
-  TDS_DISPATCH(dtype, (launch_k(ln_fwd_kernel<T>, dim3(grid), dim3(block), 0, s, (const T*)x, (const T*)w, (const T*)b, (T*)y, mean,
-                                                                rstd, M, N, eps)));
+  const bool vec = rows_vec16((int64_t)N * (dtype == kBF16 ? 2 : 4), {x, w, b, y});
+  TDS_DISPATCH(dtype, (launch_k(vec ? ln_fwd_kernel<T, true> : ln_fwd_kernel<T, false>, dim3(grid), dim3(block), 0, s, (const T*)x,
+                                (const T*)w, (const T*)b, (T*)y, mean, rstd, M, N, eps)));
 }
 
 // Backward: grid of kLnBwdCtas persistent CTAs; every warp walks rows (stride = total warps), producing dx
@@ -92,7 +94,7 @@ void layernorm_fwd(const void* x, const void* w, const void* b, void* y, float* 
 constexpr int kLnBwdCtas = 148;
 int layernorm_bwd_scratch_rows() { return kLnBwdCtas; }  // >= rows used by either backward variant
 
-template <typename T>
+template <typename T, bool VEC>
 __global__ void __launch_bounds__(kLnWarps * 32) ln_bwd_kernel(const T* __restrict__ dy, const T* __restrict__ x,
                                                               const T* __restrict__ w, const float* __restrict__ mean,
                                                               const float* __restrict__ rstd, const T* __restrict__ add,
@@ -105,7 +107,7 @@ __global__ void __launch_bounds__(kLnWarps * 32) ln_bwd_kernel(const T* __restri
   float* sdb = sdw + N;
   for (int i = lane; i < N; i += 32) { sdw[i] = 0.f; sdb[i] = 0.f; }
   __syncwarp();
-  const int nvec = N >> 3;
+  const int nvec = VEC ? N >> 3 : 0;
   const int gw = blockIdx.x * kLnWarps + wid, nw = gridDim.x * kLnWarps;
   for (int row = gw; row < M; row += nw) {
     const T* xr = x + (size_t)row * N;
@@ -181,10 +183,12 @@ void layernorm_bwd_generic(const void* dy, const void* x, const void* w, const f
                    cudaStream_t s) {
   const int ctas = kLnBwdCtas;
   const size_t smem = (size_t)kLnWarps * 2 * N * sizeof(float);
+  const bool vec = rows_vec16((int64_t)N * (dtype == kBF16 ? 2 : 4), {dy, x, w, add, dx});
   TDS_DISPATCH(dtype, {
+    auto kern = vec ? ln_bwd_kernel<T, true> : ln_bwd_kernel<T, false>;
     if (smem > 48 * 1024)
-      cudaFuncSetAttribute(ln_bwd_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    launch_k(ln_bwd_kernel<T>, dim3(ctas), dim3(kLnWarps * 32), smem, s, (const T*)dy, (const T*)x, (const T*)w, mean, rstd,
+      cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    launch_k(kern, dim3(ctas), dim3(kLnWarps * 32), smem, s, (const T*)dy, (const T*)x, (const T*)w, mean, rstd,
                                                         (const T*)add, (T*)dx, scratch, M, N);
     launch_k(ln_bwd_reduce_kernel<T>, dim3((2 * N + 127) / 128), dim3(128), 0, s, scratch, (T*)dw, (T*)db, ctas, N, accumulate ? 1 : 0);
   });
@@ -193,7 +197,7 @@ void layernorm_bwd_generic(const void* dy, const void* x, const void* w, const f
 // =====================================================================================================
 // Embedding
 // =====================================================================================================
-template <typename T>
+template <typename T, bool VEC>
 __global__ void emb_fwd_kernel(const int64_t* __restrict__ idx, const T* __restrict__ weight, const T* __restrict__ add,
                                int add_rows, T* __restrict__ out, int ntok, int dim, int64_t vocab) {
   pdl_launch(); pdl_wait();
@@ -205,7 +209,7 @@ __global__ void emb_fwd_kernel(const int64_t* __restrict__ idx, const T* __restr
   const T* src = weight + (size_t)id * dim;
   const T* ar = add ? add + (size_t)(tok % add_rows) * dim : nullptr;
   T* dst = out + (size_t)tok * dim;
-  const int nvec = dim >> 3;
+  const int nvec = VEC ? dim >> 3 : 0;
   for (int i = lane; i < nvec; i += 32) {
     float f[8];
     V8<T>::ld(src + i * 8, f);
@@ -223,8 +227,10 @@ __global__ void emb_fwd_kernel(const int64_t* __restrict__ idx, const T* __restr
 void embedding_fwd(const int64_t* idx, const void* weight, const void* add, int add_rows, void* out, int ntok, int dim,
                    int64_t vocab, int dtype, cudaStream_t s) {
   const int warps = 4;
-  TDS_DISPATCH(dtype, (launch_k(emb_fwd_kernel<T>, dim3((ntok + warps - 1) / warps), dim3(warps * 32), 0, s, 
-                          idx, (const T*)weight, (const T*)add, add_rows > 0 ? add_rows : 1, (T*)out, ntok, dim, vocab)));
+  const bool vec = rows_vec16((int64_t)dim * (dtype == kBF16 ? 2 : 4), {weight, add, out});
+  TDS_DISPATCH(dtype, (launch_k(vec ? emb_fwd_kernel<T, true> : emb_fwd_kernel<T, false>, dim3((ntok + warps - 1) / warps),
+                                dim3(warps * 32), 0, s, idx, (const T*)weight, (const T*)add, add_rows > 0 ? add_rows : 1, (T*)out,
+                                ntok, dim, vocab)));
 }
 
 TDS_DEVICE void atomic_add2(__nv_bfloat16* p, float a, float b) {
@@ -234,8 +240,12 @@ TDS_DEVICE void atomic_add2(float* p, float a, float b) {
   atomicAdd(p, a);
   atomicAdd(p + 1, b);
 }
+TDS_DEVICE void atomic_add1(__nv_bfloat16* p, float a) { atomicAdd(p, __float2bfloat16_rn(a)); }   // native on sm_90+
+TDS_DEVICE void atomic_add1(float* p, float a) { atomicAdd(p, a); }
 
-template <typename T>
+// PAIR: element pairs (i, i + 1) of every gradient row are one 4-byte __nv_bfloat162 atomic (host: even dim and a 4-byte
+// aligned dw, always for fp32, whose pair is two scalar atomics); otherwise one scalar atomic per element.
+template <typename T, bool PAIR>
 __global__ void emb_bwd_kernel(const int64_t* __restrict__ idx, const T* __restrict__ dy, T* __restrict__ dw, int ntok,
                                int dim, int64_t vocab, int64_t padding_idx) {
   pdl_launch(); pdl_wait();
@@ -246,10 +256,12 @@ __global__ void emb_bwd_kernel(const int64_t* __restrict__ idx, const T* __restr
   if (id < 0 || id >= vocab || id == padding_idx) return;
   const T* src = dy + (size_t)tok * dim;
   T* dst = dw + (size_t)id * dim;
-  for (int i = lane * 2; i + 1 < dim; i += 64) atomic_add2(dst + i, ldf(src + i), ldf(src + i + 1));
-  if ((dim & 1) && lane == 0) {
-    // odd tail: single-element CAS-free path is only needed for fp32; bf16 dims are even in practice
-    if (sizeof(T) == 4) atomicAdd(reinterpret_cast<float*>(dst) + dim - 1, ldf(src + dim - 1));
+  if (PAIR) {
+    for (int i = lane * 2; i + 1 < dim; i += 64) atomic_add2(dst + i, ldf(src + i), ldf(src + i + 1));
+    // odd tail: fp32 only, the host runs bf16 pairs for even dims only (odd bf16 dims take the scalar loop below)
+    if (sizeof(T) == 4 && (dim & 1) && lane == 0) atomic_add1(dst + dim - 1, ldf(src + dim - 1));
+  } else {
+    for (int i = lane; i < dim; i += 32) atomic_add1(dst + i, ldf(src + i));
   }
 }
 
@@ -258,8 +270,9 @@ void embedding_bwd(const int64_t* idx, const void* dy, void* dw, bool accumulate
   const size_t esz = dtype == kBF16 ? 2 : 4;
   if (!accumulate) cudaMemsetAsync(dw, 0, (size_t)vocab * dim * esz, s);
   const int warps = 4;
-  TDS_DISPATCH(dtype, (launch_k(emb_bwd_kernel<T>, dim3((ntok + warps - 1) / warps), dim3(warps * 32), 0, s, 
-                          idx, (const T*)dy, (T*)dw, ntok, dim, vocab, padding_idx)));
+  const bool pair = dtype != kBF16 || (dim % 2 == 0 && (reinterpret_cast<uintptr_t>(dw) & 3) == 0);
+  TDS_DISPATCH(dtype, (launch_k(pair ? emb_bwd_kernel<T, true> : emb_bwd_kernel<T, false>, dim3((ntok + warps - 1) / warps),
+                                dim3(warps * 32), 0, s, idx, (const T*)dy, (T*)dw, ntok, dim, vocab, padding_idx)));
 }
 
 // =====================================================================================================
@@ -362,7 +375,7 @@ void softmax_causal_bwd_generic(const void* p, void* dp_inout, int nmat, int T, 
 // =====================================================================================================
 constexpr int kXentThreads = 512;
 
-template <typename T>
+template <typename T, bool VEC>
 __global__ void __launch_bounds__(kXentThreads) xent_fwd_kernel(const T* __restrict__ logits,
                                                                 const int64_t* __restrict__ tgt,
                                                                 float* __restrict__ row_loss, float* __restrict__ lse,
@@ -371,7 +384,7 @@ __global__ void __launch_bounds__(kXentThreads) xent_fwd_kernel(const T* __restr
   __shared__ float red[32];
   const int row = blockIdx.x;
   const T* l = logits + (size_t)row * V;
-  const int nvec = V >> 3;
+  const int nvec = VEC ? V >> 3 : 0;
   float mx = -INFINITY, sum = 0.f;
   for (int i = threadIdx.x; i < nvec; i += blockDim.x) {
     float f[8];
@@ -410,11 +423,13 @@ __global__ void mean_kernel(const float* __restrict__ v, float* __restrict__ out
 
 void xent_fwd(const void* logits, const int64_t* tgt, float* row_loss, float* lse, float* loss, int M, int V, int dtype,
               cudaStream_t s) {
-  TDS_DISPATCH(dtype, (launch_k(xent_fwd_kernel<T>, dim3(M), dim3(kXentThreads), 0, s, (const T*)logits, tgt, row_loss, lse, V)));
+  const bool vec = rows_vec16((int64_t)V * (dtype == kBF16 ? 2 : 4), {logits});
+  TDS_DISPATCH(dtype, (launch_k(vec ? xent_fwd_kernel<T, true> : xent_fwd_kernel<T, false>, dim3(M), dim3(kXentThreads), 0, s,
+                                (const T*)logits, tgt, row_loss, lse, V)));
   launch_k(mean_kernel, dim3(1), dim3(1024), 0, s, row_loss, loss, M);
 }
 
-template <typename T>
+template <typename T, bool VEC>
 __global__ void __launch_bounds__(kXentThreads) xent_bwd_kernel(const T* __restrict__ logits,
                                                                 const int64_t* __restrict__ tgt,
                                                                 const float* __restrict__ lse,
@@ -426,7 +441,7 @@ __global__ void __launch_bounds__(kXentThreads) xent_bwd_kernel(const T* __restr
   T* d = dl + (size_t)row * V;
   const float z = lse[row], g = gloss[0] / M;
   const int64_t t = tgt[row];
-  const int nvec = V >> 3;
+  const int nvec = VEC ? V >> 3 : 0;
   for (int i = threadIdx.x; i < nvec; i += blockDim.x) {
     float f[8];
     V8<T>::ld(l + i * 8, f);
@@ -440,8 +455,9 @@ __global__ void __launch_bounds__(kXentThreads) xent_bwd_kernel(const T* __restr
 
 void xent_bwd(const void* logits, const int64_t* tgt, const float* lse, const float* gloss, void* dlogits, int M, int V,
               int dtype, cudaStream_t s) {
-  TDS_DISPATCH(dtype,
-               (launch_k(xent_bwd_kernel<T>, dim3(M), dim3(kXentThreads), 0, s, (const T*)logits, tgt, lse, gloss, (T*)dlogits, M, V)));
+  const bool vec = rows_vec16((int64_t)V * (dtype == kBF16 ? 2 : 4), {logits, dlogits});
+  TDS_DISPATCH(dtype, (launch_k(vec ? xent_bwd_kernel<T, true> : xent_bwd_kernel<T, false>, dim3(M), dim3(kXentThreads), 0, s,
+                                (const T*)logits, tgt, lse, gloss, (T*)dlogits, M, V)));
 }
 
 // =====================================================================================================

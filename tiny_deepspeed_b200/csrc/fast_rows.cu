@@ -162,10 +162,14 @@ static void launch_ln_bwd(const void* dy, const void* x, const void* w, const fl
     launch_k(ln_fold_kernel, dim3((2 * N + 31) / 32), dim3(256), 0, s, scratch, (__nv_bfloat16*)dw, (__nv_bfloat16*)db, ctas, N, accumulate ? 1 : 0);
 }
 
+bool layernorm_bwd_fast_ok(const void* dy, const void* x, const void* w, const void* add, const void* dx, int N, int dtype) {
+  return dtype == kBF16 && N % 8 == 0 && N <= 2048 && rows_vec16((int64_t)N * 2, {dy, x, w, add, dx});
+}
+
 void layernorm_bwd(const void* dy, const void* x, const void* w, const float* mean, const float* rstd, const void* add,
                    void* dx, float* scratch, void* dw, void* db, bool accumulate, int M, int N, int dtype,
                    cudaStream_t s, int* counter) {
-  if (dtype == kBF16 && N % 8 == 0 && N <= 2048) {
+  if (layernorm_bwd_fast_ok(dy, x, w, add, dx, N, dtype)) {
     if (N <= 1024) launch_ln_bwd<4>(dy, x, w, mean, rstd, add, dx, scratch, dw, db, accumulate, M, N, counter, s);
     else launch_ln_bwd<8>(dy, x, w, mean, rstd, add, dx, scratch, dw, db, accumulate, M, N, counter, s);
     return;

@@ -3,9 +3,22 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <initializer_list>
+
 namespace tds {
 
 enum DType : int { kBF16 = 0, kF32 = 1 };
+
+// The row kernels read and write 16 bytes at a time at `base + row * pitch + 16 * i`.  That is legal only when every row
+// starts on a 16-byte boundary: the row pitch is a multiple of 16 bytes and every base pointer (nullptr = operand absent)
+// is 16-byte aligned.  Otherwise (bf16 rows of N % 8 != 0 elements, fp32 rows of N % 4 != 0, offset views) the kernels
+// run their scalar loop over the whole row.  Decided once per launch, never per row.
+inline bool rows_vec16(int64_t row_bytes, std::initializer_list<const void*> ptrs) {
+  if (row_bytes % 16 != 0) return false;
+  for (const void* p : ptrs)
+    if (reinterpret_cast<uintptr_t>(p) & 15) return false;
+  return true;
+}
 
 // ---- GEMM (gemm_sm100.cu) ---------------------------------------------------------------------
 // D[b][m][n] = alpha * sum_k A(b,m,k) * B(b,n,k)  (+ epilogue).  bf16 (or fp32-as-TF32) operands, fp32 accumulate in TMEM.
@@ -51,6 +64,8 @@ int layernorm_bwd_scratch_rows();
 void layernorm_bwd(const void* dy, const void* x, const void* w, const float* mean, const float* rstd,
                    const void* add, void* dx, float* scratch, void* dw, void* db, bool accumulate,
                    int M, int N, int dtype, cudaStream_t s, int* counter = nullptr);   // counter: zeroed int -> single launch
+// true when layernorm_bwd takes the register-resident bf16 kernels (fast_rows.cu), the only ones that honour `counter`
+bool layernorm_bwd_fast_ok(const void* dy, const void* x, const void* w, const void* add, const void* dx, int N, int dtype);
 void embedding_fwd(const int64_t* idx, const void* weight, const void* add, int add_rows, void* out,
                    int ntok, int dim, int64_t vocab, int dtype, cudaStream_t s);
 void embedding_bwd(const int64_t* idx, const void* dy, void* dw, bool accumulate, int64_t padding_idx,
